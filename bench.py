@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: 4D-reconstruction frames/sec, 320x512x16f windows, 50-step DDIM, synthetic data.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--frames T]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--frames T] [--dump-outputs DIR]
 
 One "step" = one full pass of the hot path over a FIXED synthetic clip (default 72 frames = 8 sliding windows of
 16 frames, stride 8 -- the BASELINE.json configs[2]/[3] shape): per window VAE-encode of the 16 conditioning
@@ -16,8 +16,14 @@ single-window case for a few steps and reports it under `single_window`.
 
 `value` is timed with the video already in HBM; `e2e` includes the pinned-host -> device copy of every window's
 frames and the device -> host read of depth maps / poses / focal every step.  `--impl reference` times the
-reference's CPU path (its own modules when /root/reference is importable, else the oracle port) on a bounded
-sample of the same workload, all host threads.
+reference's CPU path (its own modules when $GEO4D_REFERENCE names its source tree, else the oracle port) on a
+bounded sample of the same workload, all host threads.
+
+`--dump-outputs DIR` writes what the last timed step returned (see dump_outputs) so that two builds can be compared
+output for output: every input -- weights, video, initial latents, the VAE posterior noise -- comes from a fixed
+seed, so the same arguments give the same inputs in every run.  The GEMM tile autotuner picks by timing, and a
+split-K choice changes rounding, which 50 DDIM steps and the alignment amplify; with GEO4D_AUTOTUNE=0 repeated
+runs of one build give bit-identical outputs.
 """
 from __future__ import annotations
 
@@ -207,12 +213,35 @@ def n_windows_of(T):
     return len(sliding_windows(T, 8))
 
 
+DUMP_MAX_PIXELS = 1 << 22   # per-pixel arrays of larger clips are sampled: 2 x 16 MB, well under 64 MB in all
+
+
+def dump_outputs(scene, out_dir):
+    """The arrays a caller of the timed path receives from the aligned scene, as out_dir/<name>.npy (float32):
+    depth maps and confidence [T, H, W], camera-to-world poses [T, 4, 4], focals [T, 1], principal points [T, 2].
+    When the clip has more than DUMP_MAX_PIXELS pixels, depth and confidence are taken at one fixed seeded sample
+    of pixel indices (sorted, flattened over T, H, W), the same in every run with the same clip shape."""
+    import numpy as np
+    import torch
+    depth = torch.stack(scene.get_depthmaps())
+    conf = torch.stack(scene.get_conf())
+    if depth.numel() > DUMP_MAX_PIXELS:
+        idx = torch.randperm(depth.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_MAX_PIXELS]
+        idx = idx.sort().values.to(depth.device)
+        depth, conf = depth.reshape(-1)[idx], conf.reshape(-1)[idx]
+    out = {"depthmaps": depth, "conf": conf, "poses": scene.get_im_poses(), "focals": scene.get_focals(),
+           "principal_points": scene.get_principal_points()}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 # ----------------------------------------------------------------------------------------------- reference arm
 def _reference_modules():
-    """The reference's own U-Net / VAE classes when its tree is importable (build container: /root/reference; a
-    box where baseline/_ref holds it), else None -> the oracle port.  Nothing is read from it on the GPU box."""
-    for root in (os.environ.get("GEO4D_REFERENCE", "/root/reference"), os.path.join(REPO, "baseline", "_ref")):
-        if os.path.isdir(os.path.join(root, "lvdm", "modules", "networks")):
+    """The reference's own U-Net / VAE classes when its tree is importable ($GEO4D_REFERENCE, or baseline/_ref in
+    this tree), else None -> the oracle port."""
+    for root in (os.environ.get("GEO4D_REFERENCE"), os.path.join(REPO, "baseline", "_ref")):
+        if root and os.path.isdir(os.path.join(root, "lvdm", "modules", "networks")):
             try:
                 sys.path.insert(0, root)
                 from oracle.gen_golden import install_shims
@@ -350,6 +379,9 @@ def run_b200(args, rank, world, local):
     from geo4d_b200 import ops, sharding, synthetic
     from geo4d_b200.pipeline import Geo4DPipeline, sliding_windows
     torch.cuda.set_device(local)
+    # the VAE encoder draws its posterior noise from the global CPU generator, which torch does not seed the same
+    # way in every process: seeded here, every run with the same arguments gets the same inputs
+    torch.manual_seed(0)
     dev = torch.device("cuda", local)
     if world > 1:
         import datetime
@@ -405,6 +437,8 @@ def run_b200(args, rank, world, local):
     launches = ops.launch_count() - n0
     phase_ms = pipe.phase_ms()
     shard_info = getattr(scene, "_shard", None)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(scene, args.dump_outputs)
     # ---- timed region 2: end to end from pinned host memory, results read back (fewer steps: same per-step work)
     e2e_steps = max(1, min(args.steps, args.e2e_steps if args.e2e_steps > 0 else max(2, args.steps // 4)))
     barrier()
@@ -539,7 +573,11 @@ def main():
     ap.add_argument("--e2e-steps", type=int, default=0, help="steps of the end-to-end region (0: max(2, steps/4))")
     ap.add_argument("--single-window-steps", type=int, default=3)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
